@@ -244,6 +244,24 @@ def bind_to_gpu_numa(index):
 
 
 RHD_RECORD_BYTES, RHD_IMAGE_OFF = 410520, 878     # data/BinaryDbReader.py:103-208 (header 876 B + 2 B pad, then 320x320x3 u8)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, result):
+    """Writes the arrays of one step's result dict as <out_dir>/<name>.npy in float32 (the int32 key-point indices are exact
+    in float32), so that two builds run with the same arguments can be compared output for output.  Above DUMP_LIMIT_BYTES
+    every array keeps the same seeded sample of images, whose indices go to sample_rows.npy."""
+    arrays = {k: v.detach().cpu().numpy().astype(np.float32) for k, v in result.items() if v is not None}
+    B = next(iter(arrays.values())).shape[0]
+    per_row = sum(a.nbytes for a in arrays.values()) // B
+    if B * per_row > DUMP_LIMIT_BYTES:
+        n = (DUMP_LIMIT_BYTES - (1 << 20)) // (per_row + 8)          # 1 MB left for the index file's and the headers' slack
+        rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def run_ours(args):
@@ -312,7 +330,8 @@ def run_ours(args):
             graph_launches[0] += nl
         else:
             r = run_stage(dev_imgs[i % NBUF], dev_hs[i % NBUF])
-        return exchange(r)
+        exchange(r)
+        return r
 
     def barrier():
         if world > 1:
@@ -352,7 +371,7 @@ def run_ours(args):
     barrier()
     e0.record()
     for i in range(args.steps):
-        step_device(i)
+        last = step_device(i)
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
@@ -360,6 +379,8 @@ def run_ours(args):
     sampler.stop_flag = True
     sampler.join(timeout=2.0)
     value = world * B * args.steps / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)      # before any later replay overwrites the graph's result buffers
 
     # ---- sustained: the same loop for several seconds (power / thermal steady state), reported beside the K-step value
     sustained = None
@@ -563,7 +584,13 @@ def main():
     ap.add_argument("--sustain-seconds", type=float, default=3.0, help="extra sustained loop after the timed K steps (0 = off)")
     ap.add_argument("--e2e-input", default="records", choices=["records", "f32"], help="what the end-to-end loop copies host -> device")
     ap.add_argument("--e2e-all-outputs", type=int, default=1, help="also time the end-to-end loop with every reference output read back")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = CONFIGS[args.config]
     for k in ("batch", "stage", "height", "width", "precision", "cuda_graph"):
         if getattr(args, k) is None:

@@ -9,7 +9,8 @@ create_multiple_gaussian_map, scale_to_size, convert_kp, canonical_trafo.  The h
 resize) are oracle/tf1_ops.py, pinned separately by tests/test_tf_published_vectors.py.
 
     python tests/golden/make_golden_reference_reader.py       # only where /root/reference exists; ~1 minute of CPU
-Large tensors (image, image_crop, scoremap) are stored as an 8x sub-sampled copy plus float64 sum / sum of squares.
+Large tensors (image, image_crop, scoremap) are stored as a sub-sampled copy plus float64 sum / sum of squares.  Score maps
+take every 16th pixel (their Gaussians have sigma = 25 px), the others every 8th, which keeps the file well under 1 MB.
 """
 import os
 import sys
@@ -51,11 +52,16 @@ def setup_imports():
 BIG = ("image", "image_crop", "scoremap", "hand_parts", "hand_mask")
 
 
+def sub_step(k):
+    return 16 if k == "scoremap" else 8
+
+
 def pack(prefix, d, out):
     for k, v in d.items():
         v = np.squeeze(np.asarray(v), 0)                  # batch_join adds the batch dimension of 1
         if k in BIG:
-            out["%s/%s/sub8" % (prefix, k)] = np.ascontiguousarray(v[::8, ::8])
+            s = sub_step(k)
+            out["%s/%s/sub%d" % (prefix, k, s)] = np.ascontiguousarray(v[::s, ::s])
             out["%s/%s/sums" % (prefix, k)] = np.array([v.astype(np.float64).sum(), np.square(v.astype(np.float64)).sum()])
             out["%s/%s/shape" % (prefix, k)] = np.array(v.shape)
         else:

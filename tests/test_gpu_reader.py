@@ -13,6 +13,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 import synth_records as SR  # noqa: E402
+from make_golden_reference_reader import sub_step  # noqa: E402
 from oracle import reader_oracle as R  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -68,9 +69,10 @@ def test_rhd_reader_mirror(tmp_path, cfg):
         for k in ("hand_side", "keypoint_xyz21", "keypoint_uv21", "keypoint_vis21", "keypoint_scale", "crop_scale"):
             if pre + "/" + k in G.files:
                 np.testing.assert_allclose(_np(d[k])[i].astype(np.float64), G[pre + "/" + k].astype(np.float64), atol=2e-6, rtol=2e-6, err_msg=k)
-        if pre + "/scoremap/sub8" in G.files:
+        if pre + "/scoremap/shape" in G.files:
             sm = _np(d["scoremap"])[i]
-            np.testing.assert_allclose(sm[::8, ::8], G[pre + "/scoremap/sub8"], atol=2e-6)
+            s = sub_step("scoremap")
+            np.testing.assert_allclose(sm[::s, ::s], G["%s/scoremap/sub%d" % (pre, s)], atol=2e-6)
             np.testing.assert_allclose(sm.astype(np.float64).sum(), G[pre + "/scoremap/sums"][0], rtol=1e-5, atol=1e-4)
 
 

@@ -104,8 +104,6 @@ def test_oracle_relative_trafo_matches_reference_graph():
 
 # ------------------------------------------------------------------------------------------- CUDA path (GPU)
 @pytest.mark.gpu
-@pytest.mark.xfail(strict=False, reason="written after the round's GPU budget was spent: runs, but its outcome has not been seen on "
-                                        "hardware yet (XPASS expected; the same stages are covered against the oracle in test_golden.py)")
 @pytest.mark.parametrize("prec,tol", [("fp32_ffma", 2e-4), ("bf16x3", 1e-3), ("fp16x3", 1e-3)])
 def test_cuda_path_matches_reference_graph(prec, tol, wd):
     """Stage-wise against the reference-graph tensors (teacher-forced inputs), plus the key-points of the whole pipeline."""

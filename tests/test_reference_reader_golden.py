@@ -10,6 +10,7 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 import synth_records as SR  # noqa: E402
+from make_golden_reference_reader import sub_step  # noqa: E402
 from oracle import reader_oracle as R  # noqa: E402
 
 G = np.load(os.path.join(HERE, "golden", "golden_reference_reader.npz"))
@@ -29,7 +30,8 @@ def check(prefix, d, atol=1e-6):
         v = np.asarray(d[k])
         if k in BIG:
             assert list(v.shape) == list(G["%s/%s/shape" % (prefix, k)]), k
-            np.testing.assert_allclose(v[::8, ::8], G["%s/%s/sub8" % (prefix, k)], atol=atol, rtol=0, err_msg=k)
+            s = sub_step(k)
+            np.testing.assert_allclose(v[::s, ::s], G["%s/%s/sub%d" % (prefix, k, s)], atol=atol, rtol=0, err_msg=k)
             sums = np.array([v.astype(np.float64).sum(), np.square(v.astype(np.float64)).sum()])
             np.testing.assert_allclose(sums, G["%s/%s/sums" % (prefix, k)], rtol=1e-7, atol=1e-6, err_msg=k)
         else:
